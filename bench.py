@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference CPU algorithms (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the last step's outputs as DIR/*.npy
 
 One "step" = one pass of the hot path over one batch of synthetic input:
   * product arm: one 2^lg-point VariableBase::msm per GPU (weak scaling: every rank owns 2^lg points;
@@ -94,6 +95,17 @@ def base_multipliers(seed, n):
     ks = np.zeros((n, 4), dtype=np.uint64)
     ks[:, 0] = k
     return ks
+
+
+def u64_as_f64(a):
+    """uint64 limbs → their little-endian 32-bit words as float64 (last axis doubles); exact, every word is < 2^32"""
+    return np.ascontiguousarray(a, dtype=np.uint64).view(np.uint32).astype(np.float64)
+
+
+def dump_outputs(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, f"{name}.npy"), a)
 
 
 def limbs_to_int(a):
@@ -365,6 +377,7 @@ def run_product(args, rank, world, local_rank):
     red_ms, _ = _lib.profile_collect(_lib.PROF_MSM_REDUCE)
     _lib.profile_enable(False)
     assert all((o == expect).all() for o in outs), "MSM result changed between steps"
+    dumps = {"msm": u64_as_f64(outs[-1])}                # normalised projective X, Y, Z (Montgomery limbs) of the last step
     ms_total = ms_per_step * args.steps
     value = n * world / (ms_per_step * 1e-3)
     acc_ms_per_step = acc_ms / max(1, args.steps)           # the whole accumulation phase of one MSM (several kernels)
@@ -476,6 +489,11 @@ def run_product(args, rank, world, local_rank):
         ntt_ms, _ = timed(lambda: device.ntt_(x, NTTDirection.Forward, NTTType.Standard, scratch), reps)
         pass_ms, pass_n = _lib.profile_collect(_lib.PROF_NTT_PASS)
         _lib.profile_enable(False)
+        if args.dump_outputs:
+            # x now holds the last timed transform's output: a fixed, seeded sample of its rows (Montgomery limbs)
+            rows = np.sort(np.random.default_rng(0).choice(nn, size=min(nn, 1 << 16), replace=False))
+            dumps["ntt_rows"] = rows.astype(np.float64)
+            dumps["ntt"] = u64_as_f64(x[torch.from_numpy(rows).to(dev)].cpu().numpy().view(np.uint64))
         xs_page = np.empty((nn, 4), dtype=np.uint64); xs_page[:] = random_scalars(nn, 5)
         xs_pin_t = torch.from_numpy(xs_page.view(np.int64).copy()).pin_memory()
         xs_pin = xs_pin_t.numpy().view(np.uint64)
@@ -678,6 +696,8 @@ def run_product(args, rank, world, local_rank):
         "g2_msm": g2_line,
         "msm_sizes": sizes_line,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumps)
     print(json.dumps(line), flush=True)
 
 
@@ -706,7 +726,15 @@ def main():
     ap.add_argument("--skip-strong", action="store_true")
     ap.add_argument("--skip-registered", action="store_true")
     ap.add_argument("--skip-precomputed", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned as DIR/<name>.npy: msm.npy (the G1 MSM result) and, "
+                         "unless --skip-ntt, ntt.npy (a seeded sample of 2^16 rows of the last timed NTT output, their indices in "
+                         "ntt_rows.npy); uint64 limbs are stored as their little-endian 32-bit words in float64, which is exact")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the product path (--impl b200)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
 

@@ -120,7 +120,4 @@ with open(os.path.join(REF, "parameters/src/mainnet/resources/powers-of-beta-15.
     blob = f.read(8 + 512 * 96)
 with open(os.path.join(OUT, "powers_of_beta_15_first512.usrs"), "wb") as f:
     f.write((512).to_bytes(8, "little") + blob[8:])
-# the whole 2^15-point file (3 MB), for lagrange_basis at a real committer-key size (kzg10/data_structures.rs:68-72)
-import shutil
-shutil.copyfile(os.path.join(REF, "parameters/src/mainnet/resources/powers-of-beta-15.usrs"), os.path.join(OUT, "powers_of_beta_15.usrs"))
 print("wrote", os.listdir(OUT))

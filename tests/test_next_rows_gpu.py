@@ -63,21 +63,40 @@ def test_lagrange_basis_real_srs_and_commit_lagrange(oracle_cpu):
         KZG10.commit_lagrange(basis, _dev(evals[:100]))       # next_power_of_two(100) != 256
 
 
-def test_lagrange_basis_of_the_whole_real_srs(oracle_cpu):
-    """UniversalParams::lagrange_basis (kzg10/data_structures.rs:68-72) of all 2^15 mainnet powers-of-beta (the reference's
-    parameters/src/mainnet/resources/powers-of-beta-15.usrs, copied by tests/golden/make_golden.py): decoded on the device, every
-    basis point equal to the oracle's group iFFT, and Σ_i L_i(β)·G = powers[0] = G."""
+def _powers_of_tau_usrs(cpu, n, tau):
+    """A .usrs file in the layout of the mainnet powers-of-beta files (u64-LE count, then per point x and y as 48-byte LE canonical
+    integers, flag bits clear) holding P_i = τ^i·G for i < n, built with the oracle's scalar multiplication."""
+    g = np.frombuffer(py.affine_bytes(py.G1_GENERATOR), dtype=np.uint8)
+    proj = np.empty((n, 18), dtype=np.uint64)
+    k = 1
+    for i in range(n):
+        proj[i] = cpu.g1_mul(g, np.array(py.to_limbs(k, 4), dtype=np.uint64))    # normalised: Z = 1, X and Y affine
+        k = k * tau % py.R_MOD
+    xy = np.concatenate([cpu.fq_from_mont(proj[:, 0:6]), cpu.fq_from_mont(proj[:, 6:12])], axis=1)
+    return n.to_bytes(8, "little") + xy.tobytes()
+
+
+def test_lagrange_basis_of_a_2_15_point_srs(oracle_cpu):
+    """UniversalParams::lagrange_basis (kzg10/data_structures.rs:68-72) at the size of the mainnet powers-of-beta-15 file, on a
+    seeded powers-of-τ SRS in the same file layout (the real points are covered by the 512-point excerpt above): decoded on the
+    device, every basis point equal to the oracle's group iFFT, Σ_i L_i(τ)·G = powers[0] = G, and a few basis points equal to
+    their closed form L_i(τ)·G = (τ^n − 1)·ω^i / (n·(τ − ω^i))·G."""
     import torch
     from snarkvm_b200 import device
-    blob = open(os.path.join(HERE, "golden", "powers_of_beta_15.usrs"), "rb").read()
-    n = int.from_bytes(blob[:8], "little")
-    assert n == 1 << 15 and len(blob) == 8 + n * 96
+    n = 1 << 15
+    tau = py.from_limbs(random_canonical_fr(1, seed=15)[0])
+    blob = _powers_of_tau_usrs(oracle_cpu, n, tau)
     powers = affine_array(py.parse_usrs_points(blob, n))
     raw = torch.from_numpy(np.frombuffer(blob[8:], dtype=np.uint8).copy()).cuda()
     decoded, invalid = device.srs_decode(raw)
     assert invalid == 0 and (decoded.cpu().numpy() == powers).all()
     basis = device.lagrange_basis(decoded).cpu().numpy().reshape(n, 104)
     assert (basis == oracle_cpu.g1_ifft(powers)).all()
+    w = py.fr_root_of_unity(n)
+    for i in (0, 1, 12345, n - 1):
+        wi = pow(w, i, py.R_MOD)
+        li = (pow(tau, n, py.R_MOD) - 1) * wi * pow(n * (tau - wi), -1, py.R_MOD) % py.R_MOD
+        assert basis[i].tobytes() == py.affine_bytes(py.g1_mul(py.G1_GENERATOR, li)), i
     ones = torch.from_numpy(np.tile(py.to_limbs(1, 4), (n, 1)).astype(np.uint64).view(np.int64)).cuda()
     total = device.msm(torch.from_numpy(basis).cuda(), ones)
     assert total.tobytes() == py.projective_bytes_normalised(py.G1_GENERATOR)
