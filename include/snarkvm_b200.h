@@ -202,6 +202,20 @@ SNARKVM_API int snarkvm_b200_fr_vec_op_device(void* d_out, const void* d_a, cons
 SNARKVM_API int snarkvm_b200_fr_vec_scalar_op_device(void* d_out, const void* d_a, const void* scalar_mont_host, size_t n, int op, void* stream);
 /* EvaluationDomain::elements (fft/domain.rs:307-309): d_out[i] = group_gen^i, i < 2^lg, Montgomery. */
 SNARKVM_API int snarkvm_b200_domain_elements_device(void* d_out, uint32_t lg, void* stream);
+/* The indexer's arithmetization of A, B, C (matrix_evals, snark/varuna/ahp/matrices.rs:138-190) in one launch.  Matrix m (0 = A,
+ * 1 = B, 2 = C) is CSR in HBM: d_row_ptr[m] = num_constraints + 1 u32 offsets, d_cols[m] = nnz[m] u32 variable indices (public
+ * first), d_vals[m] = nnz[m] Montgomery Fr; its non-zero domain K_m has 2^lg_k[m] >= nnz[m] elements.  The constraint and variable
+ * domains are the next powers of two of num_constraints and num_variables; num_public (a power of two, smaller than the variable
+ * domain) is the input domain columns are reindexed by (fft/domain.rs:322-344).  Slots past nnz[m] are the padding (1, 1, 1, 0).
+ *   mode 0 (materialise): d_io[4m + j] (K_m Montgomery Fr each) receives row, col, row_col, row_col_val for j = 0..3.
+ *   mode 1 (evaluate):    d_io[m] holds the Lagrange coefficients of K_m at a point (evaluate_all_lagrange_coefficients);
+ *                         sums_mont_host (HOST, 12 x 32 B) receives sum_k L_k * e_j(k) at index 4m + j, the verifier's
+ *                         evaluate_index_polynomials (ahp/indexer/indexer.rs:232-260), without storing the evaluations.
+ * A malformed row_ptr, a column >= num_variables or nnz[m] > 2^lg_k[m] returns cudaErrorInvalidValue.  Synchronises the stream. */
+SNARKVM_API int snarkvm_b200_index_arithmetize_device(int mode, const void* const* d_row_ptr, const void* const* d_cols,
+                                                      const void* const* d_vals, const size_t* nnz, const uint32_t* lg_k,
+                                                      size_t num_constraints, size_t num_variables, size_t num_public, void* const* d_io,
+                                                      void* sums_mont_host, void* stream);
 /* DensePolynomial::evaluate (fft/polynomial/dense.rs:98-114): out = sum c_i * point^i; out and point are 32-byte HOST buffers. */
 SNARKVM_API int snarkvm_b200_poly_evaluate_device(void* out_mont_host, const void* d_coeffs, size_t m, const void* point_mont_host,
                                                   void* stream);

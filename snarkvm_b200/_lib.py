@@ -31,6 +31,7 @@ SYMBOLS = (
     "snarkvm_b200_msm_batch_device", "snarkvm_b200_msm_window_sums_plan_device", "snarkvm_b200_kzg_commit_batch_hiding_device",
     "snarkvm_b200_kzg_commit_batch_precomputed_device", "snarkvm_b200_msm_scratch_stats", "snarkvm_b200_msm_set_scratch_limit", "snarkvm_b200_msm_window_sums_host", "snarkvm_b200_selftest_coop", "snarkvm_b200_msm_plan_levels", "snarkvm_b200_msm_g2", "snarkvm_b200_msm_g2_device", "snarkvm_b200_generate_bases_g2_device",
     "snarkvm_b200_sonic_commit_batch_device", "snarkvm_b200_generator_mul_device", "snarkvm_b200_selftest_host_copy",
+    "snarkvm_b200_index_arithmetize_device",
 )
 
 
@@ -109,6 +110,7 @@ def lib():
     L.snarkvm_b200_fr_vec_op_device.argtypes = [vp, vp, vp, sz, i32, vp]
     L.snarkvm_b200_fr_vec_scalar_op_device.argtypes = [vp, vp, vp, sz, i32, vp]
     L.snarkvm_b200_domain_elements_device.argtypes = [vp, u32, vp]
+    L.snarkvm_b200_index_arithmetize_device.argtypes = [i32, vp, vp, vp, vp, vp, sz, sz, sz, vp, vp, vp]
     L.snarkvm_b200_msm_batch_device.argtypes = [vp, vp, sz, vp, vp, sz, vp]
     L.snarkvm_b200_msm_window_sums_plan_device.argtypes = [vp, vp, sz, vp, sz, vp, sz, vp]
     L.snarkvm_b200_kzg_commit_batch_hiding_device.argtypes = [vp, vp, sz, vp, vp, vp, vp, vp, sz, vp]

@@ -1152,6 +1152,12 @@ int snarkvm_b200_fr_vec_scalar_op_device(void* d_out, const void* d_a, const voi
 int snarkvm_b200_domain_elements_device(void* d_out, uint32_t lg, void* stream) {
     return domain_elements_device(d_out, lg, (cudaStream_t)stream);
 }
+int snarkvm_b200_index_arithmetize_device(int mode, const void* const* d_row_ptr, const void* const* d_cols, const void* const* d_vals,
+                                          const size_t* nnz, const uint32_t* lg_k, size_t num_constraints, size_t num_variables,
+                                          size_t num_public, void* const* d_io, void* sums_mont_host, void* stream) {
+    return index_arithmetize_device(mode, d_row_ptr, d_cols, d_vals, nnz, lg_k, num_constraints, num_variables, num_public, d_io,
+                                    sums_mont_host, (cudaStream_t)stream);
+}
 int snarkvm_b200_poly_evaluate_device(void* out_mont_host, const void* d_coeffs, size_t m, const void* point_mont_host, void* stream) {
     return poly_evaluate_device(out_mont_host, d_coeffs, m, point_mont_host, (cudaStream_t)stream);
 }

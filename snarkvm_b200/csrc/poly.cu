@@ -418,6 +418,164 @@ __global__ void k_domain_elements(uint32_t* __restrict__ out, int lg, const uint
     (i < half ? w : w.neg()).store(out + i * 8);
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// The indexer's arithmetization of A, B, C (matrix_evals, snark/varuna/ahp/matrices.rs:138-190) in one launch: thread κ of
+// matrix m (blockIdx.y) finds its entry's row by a binary search in row_ptr, remaps the column with reindex_by_subdomain
+// (fft/domain.rs:322-344) and reads ω_R^row, ω_C^col from the NTT twiddle table, so no per-entry index array and no |R| or
+// |C| element table exists.  Slots κ ≥ nnz_m are the padding (1, 1, 1, 0).
+//   INDEX_MATERIALISE: the four evaluation vectors row, col, row_col = row·col, row_col_val = val·row_col on K_m.
+//   INDEX_EVALUATE:    Σ_κ L_κ(z)·e(κ) for the four vectors (MatrixEvals::evaluate with the Lagrange coefficients of K_m at z,
+//                      ahp/indexer/indexer.rs:232-260): CTA partial sums, then one CTA per sum adds the partials.
+// A row_ptr that is not a CSR offset array over nnz_m entries, or a column ≥ num_variables, sets *bad; the entry is skipped.
+// ---------------------------------------------------------------------------------------------------------------------
+struct IndexMatrix {
+    const uint32_t* row_ptr;     // nrows + 1
+    const uint32_t* cols;        // nnz
+    const uint32_t* vals;        // nnz Montgomery Fr
+    uint32_t* out[4];            // INDEX_MATERIALISE: row, col, row_col, row_col_val [K]
+    const uint32_t* lagrange;    // INDEX_EVALUATE: L_κ(z) [K]
+    uint32_t nnz, lg_k;
+};
+struct IndexArgs {
+    IndexMatrix m[3];
+    const uint32_t* tw;          // ω_N^j, j < N/2
+    uint32_t nrows, num_variables, num_public;
+    int lg_r, lg_c, lgN;
+};
+FF_DEV Fr domain_element(const uint32_t* tw, int lgN, int lg, uint64_t i) {     // ω_n^i, n = 2^lg (as k_domain_elements)
+    if (lg == 0) return Fr::one();
+    const uint64_t half = (uint64_t)1 << (lg - 1), j = i < half ? i : i - half;
+    const Fr w = Fr::load_ldg(tw + (j << (lgN - lg)) * 8);
+    return i < half ? w : w.neg();
+}
+template <int MODE>
+__global__ void __launch_bounds__(EVAL_THREADS) k_index_arith(IndexArgs a, uint32_t* __restrict__ partial, uint32_t max_blocks,
+                                                               int* __restrict__ bad) {
+    const IndexMatrix& M = a.m[blockIdx.y];
+    const uint64_t k = (uint64_t)blockIdx.x * EVAL_THREADS + threadIdx.x, K = (uint64_t)1 << M.lg_k;
+    Fr e[4] = {Fr::one(), Fr::one(), Fr::one(), Fr::zero()};
+    if (k < M.nnz) {
+        uint32_t lo = 0, hi = a.nrows;                                  // largest r < nrows with row_ptr[r] ≤ κ
+        while (hi - lo > 1) {
+            const uint32_t mid = lo + (hi - lo) / 2;
+            if (M.row_ptr[mid] <= k) lo = mid; else hi = mid;
+        }
+        const uint32_t c = M.cols[k];
+        if (M.row_ptr[lo] > k || M.row_ptr[lo + 1] <= k || c >= a.num_variables) {
+            *bad = 1;
+        } else {
+            const uint64_t period = ((uint64_t)1 << a.lg_c) / a.num_public;
+            uint64_t ci;
+            if (c < a.num_public) {
+                ci = (uint64_t)c * period;
+            } else {
+                const uint64_t i = c - a.num_public;
+                ci = i + i / (period - 1) + 1;
+            }
+            e[0] = domain_element(a.tw, a.lgN, a.lg_r, lo);
+            e[1] = domain_element(a.tw, a.lgN, a.lg_c, ci);
+            e[2] = e[0] * e[1];
+            e[3] = Fr::load_ldg(M.vals + k * 8) * e[2];
+        }
+    }
+    if (k == 0 && M.row_ptr[a.nrows] != M.nnz) *bad = 1;
+    if constexpr (MODE == INDEX_MATERIALISE) {
+        if (k < K) {
+#pragma unroll
+            for (int j = 0; j < 4; j++) e[j].store(M.out[j] + k * 8);
+        }
+    } else {
+        __shared__ uint4 sh4[EVAL_THREADS * 2];
+        const Fr l = k < K ? Fr::load_ldg(M.lagrange + k * 8) : Fr::zero();
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const Fr s = cta_sum(e[j] * l, reinterpret_cast<uint32_t*>(sh4));
+            if (threadIdx.x == 0) s.store(partial + (((size_t)blockIdx.y * max_blocks + blockIdx.x) * 4 + j) * 8);
+            __syncthreads();
+        }
+    }
+}
+// CTA (m, j) adds the partial sums of vector j of matrix m
+__global__ void __launch_bounds__(EVAL_THREADS) k_index_sums(const uint32_t* __restrict__ partial, uint32_t max_blocks, uint3 nblocks,
+                                                             uint32_t* __restrict__ out) {
+    __shared__ uint4 sh4[EVAL_THREADS * 2];
+    const uint32_t m = blockIdx.x / 4, j = blockIdx.x % 4, nb = m == 0 ? nblocks.x : m == 1 ? nblocks.y : nblocks.z;
+    Fr acc = Fr::zero();
+    for (uint32_t b = threadIdx.x; b < nb; b += EVAL_THREADS) acc = acc + Fr::load_ldg(partial + (((size_t)m * max_blocks + b) * 4 + j) * 8);
+    const Fr s = cta_sum(acc, reinterpret_cast<uint32_t*>(sh4));
+    if (threadIdx.x == 0) s.store(out + blockIdx.x * 8);
+}
+
+int index_arithmetize_device(int mode, const void* const* d_row_ptr, const void* const* d_cols, const void* const* d_vals, const size_t* nnz,
+                             const uint32_t* lg_k, size_t num_constraints, size_t num_variables, size_t num_public, void* const* d_io,
+                             void* sums_mont_host, cudaStream_t stream) {
+    if ((mode != INDEX_MATERIALISE && mode != INDEX_EVALUATE) || !d_row_ptr || !d_cols || !d_vals || !nnz || !lg_k || !d_io)
+        return (int)cudaErrorInvalidValue;
+    if (mode == INDEX_EVALUATE && !sums_mont_host) return (int)cudaErrorInvalidValue;
+    // the three domains: R ⊇ rows, C ⊇ variables, X = the padded public variables, a proper subgroup of C (domain.rs:323)
+    int lg_r = 0, lg_c = 0;
+    while (((size_t)1 << lg_r) < num_constraints) lg_r++;
+    while (((size_t)1 << lg_c) < num_variables) lg_c++;
+    if (num_constraints == 0 || num_constraints > ((size_t)1 << 31) || num_variables > ((size_t)1 << 31) || lg_r > 30 || lg_c > 30)
+        return (int)cudaErrorInvalidValue;
+    if (num_public == 0 || (num_public & (num_public - 1)) || num_public >= ((size_t)1 << lg_c)) return (int)cudaErrorInvalidValue;
+    IndexArgs a{};
+    uint32_t max_blocks = 1;
+    for (int m = 0; m < 3; m++) {
+        if (lg_k[m] > 30 || nnz[m] > ((size_t)1 << lg_k[m]) || !d_row_ptr[m] || (nnz[m] && (!d_cols[m] || !d_vals[m]))) return (int)cudaErrorInvalidValue;
+        IndexMatrix& M = a.m[m];
+        M.row_ptr = (const uint32_t*)d_row_ptr[m]; M.cols = (const uint32_t*)d_cols[m]; M.vals = (const uint32_t*)d_vals[m];
+        M.nnz = (uint32_t)nnz[m]; M.lg_k = lg_k[m];
+        if (mode == INDEX_MATERIALISE) {
+            for (int j = 0; j < 4; j++) {
+                if (!d_io[m * 4 + j]) return (int)cudaErrorInvalidValue;
+                M.out[j] = (uint32_t*)d_io[m * 4 + j];
+            }
+        } else {
+            if (!d_io[m]) return (int)cudaErrorInvalidValue;
+            M.lagrange = (const uint32_t*)d_io[m];
+        }
+        const uint32_t blocks = (uint32_t)((((size_t)1 << lg_k[m]) + EVAL_THREADS - 1) / EVAL_THREADS);
+        if (blocks > max_blocks) max_blocks = blocks;
+    }
+    const void* tw = nullptr;
+    int lgN = 0, rc = 0;
+    if ((rc = ntt_get_twiddles(lg_r > lg_c ? lg_r : lg_c > 0 ? lg_c : 1, &tw, &lgN)) != 0) return rc;
+    a.tw = (const uint32_t*)tw; a.lgN = lgN; a.lg_r = lg_r; a.lg_c = lg_c;
+    a.nrows = (uint32_t)num_constraints; a.num_variables = (uint32_t)num_variables; a.num_public = (uint32_t)num_public;
+    // scratch: [0] bad flag, then (EVALUATE) 3 × max_blocks × 4 partial sums and the 12 results
+    const size_t off_partial = 256, off_sums = off_partial + (size_t)3 * max_blocks * 4 * 32;
+    uint8_t* scratch = nullptr;
+    cudaError_t e = pool_alloc(&scratch, mode == INDEX_EVALUATE ? off_sums + 12 * 32 : off_partial, stream);
+    if (e != cudaSuccess) return (int)e;
+    int* bad = (int*)scratch;
+    uint32_t* partial = (uint32_t*)(scratch + off_partial);
+    rc = (int)cudaMemsetAsync(scratch, 0, 256, stream);
+    const dim3 grid(max_blocks, 3);
+    if (rc != 0) {
+        // the flag could not be cleared: launch nothing
+    } else if (mode == INDEX_MATERIALISE) {
+        k_index_arith<INDEX_MATERIALISE><<<grid, EVAL_THREADS, 0, stream>>>(a, partial, max_blocks, bad);
+        count_launch();
+    } else {
+        uint3 nb;
+        nb.x = (uint32_t)((((size_t)1 << lg_k[0]) + EVAL_THREADS - 1) / EVAL_THREADS);
+        nb.y = (uint32_t)((((size_t)1 << lg_k[1]) + EVAL_THREADS - 1) / EVAL_THREADS);
+        nb.z = (uint32_t)((((size_t)1 << lg_k[2]) + EVAL_THREADS - 1) / EVAL_THREADS);
+        k_index_arith<INDEX_EVALUATE><<<grid, EVAL_THREADS, 0, stream>>>(a, partial, max_blocks, bad);
+        k_index_sums<<<12, EVAL_THREADS, 0, stream>>>(partial, max_blocks, nb, (uint32_t*)(scratch + off_sums));
+        count_launch(2);
+    }
+    if (rc == 0) rc = (int)cudaGetLastError();
+    int h_bad = 0;
+    if (rc == 0) rc = (int)cudaMemcpyAsync(&h_bad, bad, sizeof(int), cudaMemcpyDeviceToHost, stream);
+    if (rc == 0 && mode == INDEX_EVALUATE) rc = (int)cudaMemcpyAsync(sums_mont_host, scratch + off_sums, 12 * 32, cudaMemcpyDeviceToHost, stream);
+    cudaFreeAsync(scratch, stream);
+    if (rc == 0) rc = (int)cudaStreamSynchronize(stream);
+    if (rc == 0 && h_bad) rc = (int)cudaErrorInvalidValue;
+    return rc;
+}
+
 int fr_vec_op_device(void* d_out, const void* d_a, const void* d_b, size_t n, int op, cudaStream_t stream) {
     if (n == 0) return 0;
     if (!d_out || !d_a || !d_b || op < 0 || op > 2) return (int)cudaErrorInvalidValue;

@@ -29,6 +29,19 @@ int fr_vec_scalar_op_device(void* d_out, const void* d_a, const void* scalar_mon
 // out[i] = ω_n^i, i < n = 2^lg (EvaluationDomain::elements, fft/domain.rs:307-309)
 int domain_elements_device(void* d_out, uint32_t lg, cudaStream_t stream);
 
+// The indexer's arithmetization of A, B, C (ahp/matrices.rs:138-190) in one launch.  Per matrix m: CSR row_ptr (num_constraints + 1
+// u32), cols (nnz[m] u32 variable indices, public first), vals (nnz[m] Montgomery Fr), K_m = 2^lg_k[m] ≥ nnz[m].  The constraint
+// and variable domains are the next powers of two of num_constraints and num_variables; num_public (a power of two, smaller than
+// the variable domain) is the input domain columns are reindexed by.
+//   INDEX_MATERIALISE: d_io[4m + j] receives vector j ∈ (row, col, row_col, row_col_val) of matrix m, K_m Montgomery Fr.
+//   INDEX_EVALUATE:    d_io[m] holds the Lagrange coefficients of K_m at a point (K_m Montgomery Fr); sums_mont_host (HOST,
+//                      12 × 32 B) receives Σ_κ L_κ·e_j(κ) in the order 4m + j.
+// A malformed row_ptr or a column ≥ num_variables returns cudaErrorInvalidValue.  Synchronises the stream.
+enum { INDEX_MATERIALISE = 0, INDEX_EVALUATE = 1 };
+int index_arithmetize_device(int mode, const void* const* d_row_ptr, const void* const* d_cols, const void* const* d_vals, const size_t* nnz,
+                             const uint32_t* lg_k, size_t num_constraints, size_t num_variables, size_t num_public, void* const* d_io,
+                             void* sums_mont_host, cudaStream_t stream);
+
 // Group FFT over G1 (DomainCoeff = G1Projective, fft/domain.rs:169-221 generic path): n = 2^lg affine points in, affine points
 // out (natural order both sides).  direction 1 = inverse (includes n^{-1}): UniversalParams::lagrange_basis
 // (polycommit/kzg10/data_structures.rs:68-72).

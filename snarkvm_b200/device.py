@@ -376,6 +376,61 @@ def domain_elements(lg: int, device="cuda") -> torch.Tensor:
     return out
 
 
+INDEX_MATERIALISE, INDEX_EVALUATE = 0, 1
+
+
+def index_arithmetize(matrices: list, k_sizes: list, num_variables: int, num_public: int, lagrange: list | None = None):
+    """The indexer's arithmetization of A, B, C (matrix_evals, ahp/matrices.rs:138-190) in one launch.
+    `matrices`: three (row_ptr int32 [nrows + 1], cols int32 [nnz], vals [nnz, 4] i64 Montgomery) CUDA tensors with the same nrows;
+    `k_sizes`: the three non-zero domain sizes (powers of two ≥ nnz); `num_public`: the input domain size (a power of two below the
+    variable domain's size).
+    Without `lagrange`: → per matrix the CUDA tensors (row, col, row_col, row_col_val) [K, 4] i64 Montgomery.
+    With `lagrange` (per matrix the Lagrange coefficients of K at a point, [K, 4] Montgomery): → the twelve sums Σ_κ L_κ·e(κ) as
+    Montgomery uint64 [3, 4, 4] on the host (matrix, vector), without storing the evaluations (indexer.rs:232-260)."""
+    if len(matrices) != 3 or len(k_sizes) != 3:
+        raise ValueError("three matrices (A, B, C) and three non-zero domain sizes")
+    nrows = matrices[0][0].numel() - 1
+    if nrows < 1:
+        raise ValueError("a circuit needs at least one constraint")
+    if num_public < 1 or num_public & (num_public - 1):
+        raise ValueError("the number of public variables must be a power of two")
+    if num_public >= 1 << max(num_variables - 1, 0).bit_length():
+        raise ValueError("the input domain must be smaller than the variable domain")
+    lg_k, nnz = [], []
+    for (row_ptr, cols, vals), k in zip(matrices, k_sizes):
+        if row_ptr.dtype != torch.int32 or cols.dtype != torch.int32:
+            raise TypeError("row_ptr and cols must be int32 tensors")
+        if row_ptr.numel() - 1 != nrows:
+            raise ValueError("A, B and C must have the same number of rows")
+        n = cols.numel()
+        if _nbytes(vals) != 32 * n:
+            raise ValueError("one value per column index")
+        if k < 1 or k & (k - 1) or n > k:
+            raise ValueError(f"non-zero domain of size {k} cannot hold {n} entries")
+        lg_k.append(k.bit_length() - 1)
+        nnz.append(n)
+    dev = matrices[0][0].device
+    rp = (ctypes.c_void_p * 3)(*[_check(m[0], "row_ptr") for m in matrices])
+    cp = (ctypes.c_void_p * 3)(*[(_check(m[1], "cols") if n else None) for m, n in zip(matrices, nnz)])
+    vp = (ctypes.c_void_p * 3)(*[(_check(m[2], "vals") if n else None) for m, n in zip(matrices, nnz)])
+    nz = (ctypes.c_size_t * 3)(*nnz)
+    lk = (ctypes.c_uint32 * 3)(*lg_k)
+    if lagrange is None:
+        outs = [tuple(torch.empty((k, 4), dtype=torch.int64, device=dev) for _ in range(4)) for k in k_sizes]
+        io = (ctypes.c_void_p * 12)(*[t.data_ptr() for o in outs for t in o])
+        sums = None
+    else:
+        if len(lagrange) != 3 or any(_nbytes(l) != 32 * k for l, k in zip(lagrange, k_sizes)):
+            raise ValueError("one Lagrange coefficient vector of |K| elements per matrix")
+        io = (ctypes.c_void_p * 3)(*[_check(l, "lagrange") for l in lagrange])
+        sums = np.zeros((3, 4, 4), dtype=np.uint64)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().snarkvm_b200_index_arithmetize_device(
+            INDEX_MATERIALISE if lagrange is None else INDEX_EVALUATE, rp, cp, vp, nz, lk, nrows, num_variables, num_public, io,
+            sums.ctypes.data if sums is not None else None, _stream()))
+    return outs if lagrange is None else sums
+
+
 def sparse_matvec(row_ptr: torch.Tensor, cols: torch.Tensor, vals: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
     """z_M = M·x for a CSR matrix over Fr (inner_product per row, varuna/ahp/prover/round_functions/mod.rs:130-189).
     row_ptr: int32 [nrows + 1], cols: int32 [nnz], vals: [nnz, 4] i64 Montgomery, x: [nvars, 4] i64 Montgomery → [nrows, 4] i64."""

@@ -3,7 +3,9 @@
 Device-side mirror of /root/reference/algorithms/src/snark/varuna for the part of `prove_batch` (varuna.rs:336-620) that is
 bulk field arithmetic — the five `AHPForR1CS::prover_*_round` functions and the indexer's arithmetization:
 
-    ahp/indexer/indexer.rs:121-200, ahp/matrices.rs:138-190, 239-254   Circuit            (domains, row / col / row_col_val on K, transposes)
+    ahp/indexer/indexer.rs:121-200, ahp/matrices.rs:138-190, 239-254   Circuit            (domains, row / col / row_col / row_col_val on K, transposes)
+    ahp/indexer/circuit.rs:109-148, varuna.rs:72-134, 236-331           circuit setup      (info, id, index polynomials, batch_circuit_setup, prove_vk,
+                                                                                         evaluate_index_polynomials)
     ahp/prover/round_functions/mod.rs:43-192, ahp/prover/state.rs:107-178   init_prover   (z_A, z_B, z_C by sparse mat-vec, x_poly)
     ahp/prover/round_functions/first.rs:129-160    prover_first_round   (w)
     ahp/prover/round_functions/third.rs:207-234    calculate_assignments (z)
@@ -22,11 +24,16 @@ Polynomials are CUDA tensors [m, 4] int64 (Montgomery Fr, low degree first, NOT 
 """
 from __future__ import annotations
 
+import hashlib
+import struct
+from dataclasses import astuple, dataclass
+
 import numpy as np
 import torch
 
 from . import device
 from .algorithms import EvaluationDomain, _fr_int_to_mont, _fr_mont_to_int
+from .sonic_pc import CommitterKey, LabeledPolynomial, Randomness, SonicKZG10
 
 R_MOD = 8444461749428370424248824938781546531375899335154063827935233455917409239041   # curves/src/bls12_377/fr.rs:138-145
 
@@ -141,15 +148,74 @@ class Matrix:
 
 
 class MatrixEvals:
-    """ahp/matrices.rs:102-136: row, col, row_col_val evaluations on the non-zero domain K"""
+    """ahp/matrices.rs:102-136: row, col, row_col, row_col_val evaluations on the non-zero domain K"""
 
-    def __init__(self, row, col, row_col_val, domain):
-        self.row, self.col, self.row_col_val, self.domain = row, col, row_col_val, domain
+    def __init__(self, row, col, row_col, row_col_val, domain):
+        self.row, self.col, self.row_col, self.row_col_val, self.domain = row, col, row_col, row_col_val, domain
+
+    def vectors(self) -> tuple:
+        return self.row, self.col, self.row_col, self.row_col_val
+
+
+@dataclass(frozen=True)
+class CircuitInfo:
+    """ahp/indexer/circuit_info.rs:25-38"""
+    num_public_inputs: int
+    num_public_and_private_variables: int
+    num_constraints: int
+    num_non_zero_a: int
+    num_non_zero_b: int
+    num_non_zero_c: int
+
+    def to_bytes(self) -> bytes:
+        """the uncompressed serialisation (derive(CanonicalSerialize)): six u64, little-endian"""
+        return struct.pack("<6Q", *astuple(self))
+
+    def max_degree(self, hiding: bool) -> int:
+        """AHPForR1CS::max_degree (ahp/ahp.rs:85-108) with zk_bound 1 in the hiding mode"""
+        zk = 1 if hiding else 0
+        size = EvaluationDomain.compute_size_of_domain
+        r, v = size(self.num_constraints), size(self.num_public_and_private_variables)
+        k = size(max(self.num_non_zero_a, self.num_non_zero_b, self.num_non_zero_c))
+        return max(2 * r + 2 * zk - 2, 2 * v + 2 * zk - 2, v + 3 if hiding else 0, v, r, k - 1)
+
+    def degree_bounds(self) -> list:
+        """AHPForR1CS::get_degree_bounds (ahp/ahp.rs:110-121): |C| − 2 and |K_M| − 2"""
+        size = EvaluationDomain.compute_size_of_domain
+        bounds = [size(n) - 2 for n in (self.num_public_and_private_variables, self.num_non_zero_a, self.num_non_zero_b, self.num_non_zero_c)]
+        if min(bounds) < 0:
+            raise ValueError("every non-zero domain needs at least two elements to bound the degree of its g polynomial")
+        return bounds
+
+
+def _matrix_bytes(m: Matrix) -> bytes:
+    """Matrix<F> = Vec<Vec<(F, usize)>> serialised uncompressed (utilities/src/serialize/impls.rs:151-160, 392-420, 524-550 and
+    fields/src/macros.rs:191-): u64 row count; per row a u64 entry count, then per entry the value as 32 canonical little-endian
+    bytes and its column as u64."""
+    entries = np.zeros((m.nnz, 40), dtype=np.uint8)
+    if m.nnz:
+        entries[:, :32] = device.fr_from_mont(m.vals).cpu().numpy().view(np.uint8).reshape(m.nnz, 32)
+        entries[:, 32:] = m.cols_h.astype("<u8").view(np.uint8).reshape(m.nnz, 8)
+    body = np.empty(m.nrows * 8 + m.nnz * 40, dtype=np.uint8)
+    header = np.zeros(body.size, dtype=bool)                          # row r's count sits after r counts and row_ptr[r] entries
+    header[((np.arange(m.nrows) * 8 + m.row_ptr_h[:-1] * 40)[:, None] + np.arange(8)).ravel()] = True
+    body[header] = np.diff(m.row_ptr_h).astype("<u8").view(np.uint8)
+    body[~header] = entries.ravel()
+    return struct.pack("<Q", m.nrows) + body.tobytes()
+
+
+def index_polynomial_labels(circuit_id) -> list:
+    """AHPForR1CS::index_polynomial_labels (ahp/indexer/indexer.rs:104-122) for matrices a, b, c, in the indexer's order; the id is
+    printed as lowercase hex (ahp/indexer/circuit.rs:42-48)"""
+    cid = circuit_id.hex() if isinstance(circuit_id, (bytes, bytearray)) else str(circuit_id)
+    return [f"circuit_{cid}_{poly}_{m}" for m in "abc" for poly in ("row", "col", "row_col", "row_col_val")]
 
 
 class Circuit:
-    """AHPForR1CS::index_helper (ahp/indexer/indexer.rs:121-200) for the non-hiding mode: the caller has already padded the public
-    variables to a power of two (pad_input_for_indexer_and_prover, ahp/matrices.rs:85-100)."""
+    """AHPForR1CS::index_helper (ahp/indexer/indexer.rs:121-200): the caller has already padded the public variables to a power of
+    two (pad_input_for_indexer_and_prover, ahp/matrices.rs:85-100) and, for the hiding mode, added the randomizing variables and
+    their constraint before that (add_randomizing_variables, ahp/matrices.rs:64-82).  The arithmetization of A, B, C is one
+    device launch (device.index_arithmetize)."""
 
     def __init__(self, a: Matrix, b: Matrix, c: Matrix, num_public: int, num_variables: int):
         dev = a.vals.device
@@ -162,23 +228,13 @@ class Circuit:
         self.input_domain = EvaluationDomain.new(num_public)
         self.non_zero_domains = [EvaluationDomain.new(m.nnz) for m in (a, b, c)]
         self.max_non_zero_domain = max(self.non_zero_domains, key=lambda d: d.size)
-        r_el = device.domain_elements(self.constraint_domain.log_size_of_group, dev)
-        c_el = device.domain_elements(self.variable_domain.log_size_of_group, dev)
-        one = torch.from_numpy(_mont(1).view(np.int64)).to(dev)
+        self._id = None
         self.ariths, self.transposes = [], []
-        for m, K in zip((a, b, c), self.non_zero_domains):
+        evals = device.index_arithmetize(self._csr(), [K.size for K in self.non_zero_domains], num_variables, num_public)
+        for m, K, e in zip((a, b, c), self.non_zero_domains, evals):
+            self.ariths.append(MatrixEvals(*e, K))                                              # matrix_evals (ahp/matrices.rs:138-190)
             entry_rows = np.repeat(np.arange(m.nrows, dtype=np.int64), np.diff(m.row_ptr_h))
             entry_cols = reindex_by_subdomain(self.variable_domain.size, self.input_domain.size, m.cols_h)
-            # matrix_evals (ahp/matrices.rs:138-190)
-            row = one.repeat(K.size, 1)
-            col = one.repeat(K.size, 1)
-            rcv = _zeros(K.size, dev)
-            if m.nnz:
-                row[: m.nnz] = r_el[torch.from_numpy(entry_rows).to(dev)]
-                col[: m.nnz] = c_el[torch.from_numpy(entry_cols).to(dev)]
-                rc = device.fr_vec_op(row[: m.nnz].contiguous(), col[: m.nnz].contiguous(), device.FR_MUL)
-                rcv[: m.nnz] = device.fr_vec_op(m.vals, rc, device.FR_MUL)
-            self.ariths.append(MatrixEvals(row, col, rcv, K))
             # transpose (ahp/matrices.rs:239-254) as CSR over the variable domain's indices; entries keep the row-major order
             order = np.argsort(entry_cols, kind="stable")
             counts = np.bincount(entry_cols, minlength=self.variable_domain.size)
@@ -190,6 +246,33 @@ class Circuit:
             tm.cols = torch.from_numpy(entry_rows[order].astype(np.int32)).to(dev)
             tm.vals = t_vals.contiguous()
             self.transposes.append(tm)
+
+    def _csr(self) -> list:
+        return [(m.row_ptr, m.cols, m.vals) for m in (self.a, self.b, self.c)]
+
+    def info(self) -> CircuitInfo:
+        """CircuitInfo of the index (ahp/indexer/indexer.rs:169-176)"""
+        return CircuitInfo(self.num_public, self.num_variables, self.num_constraints, self.a.nnz, self.b.nnz, self.c.nnz)
+
+    def id(self) -> bytes:
+        """Circuit::hash (ahp/indexer/circuit.rs:109-121): Blake2s-256 over the uncompressed serialisation of the info and of A, B, C"""
+        if self._id is None:
+            h = hashlib.blake2s(digest_size=32)
+            h.update(self.info().to_bytes())
+            for m in (self.a, self.b, self.c):
+                h.update(_matrix_bytes(m))
+            self._id = h.digest()
+        return self._id
+
+    def interpolate_matrix_evals(self) -> list:
+        """Circuit::interpolate_matrix_evals (ahp/indexer/circuit.rs:142-148, MatrixArithmetization::new, ahp/matrices.rs:213-240): the
+        twelve index polynomials — the iFFT over K_M of row, col, row_col, row_col_val for M = A, B, C — with no degree or hiding
+        bound, in the indexer's label order"""
+        polys = []
+        for arith in self.ariths:
+            for v in arith.vectors():
+                polys.append(v.clone() if arith.domain.size == 1 else arith.domain.ifft(v))      # a one-point iFFT is the identity
+        return [LabeledPolynomial(label, p) for label, p in zip(index_polynomial_labels(self.id()), polys)]
 
 
 class Prover:
@@ -434,3 +517,102 @@ def test_circuit_csr(a: int, b: int, mul_depth: int, num_constraints: int, num_v
     z[padded:] = _mont(a)
     z[vb] = _mont(b)
     return circuit, torch.from_numpy(z.view(np.int64)).to(dev)
+
+
+# ---- circuit setup and the key certificate (varuna.rs:72-134, 236-331) ----
+@dataclass
+class VerifyingKey:
+    """CircuitVerifyingKey: the circuit info, the twelve index commitments (uint64 [12, 18], normalised projective) sorted by label,
+    and the circuit id"""
+    circuit_info: CircuitInfo
+    circuit_commitments: np.ndarray
+    id: bytes
+
+
+@dataclass
+class ProvingKey:
+    """CircuitProvingKey: the verifying key, the indexed circuit and the committer key trimmed for it"""
+    circuit_verifying_key: VerifyingKey
+    circuit: Circuit
+    committer_key: CommitterKey
+
+
+def batch_circuit_setup(pp_powers_of_beta_g: torch.Tensor, pp_powers_of_beta_times_gamma_g: torch.Tensor, circuits: list,
+                        hiding: bool = False) -> list:
+    """Varuna::batch_circuit_setup (varuna.rs:72-134) → [(ProvingKey, VerifyingKey)] per circuit.  Each circuit's committer key is
+    trimmed as the reference does (max_degree, hiding bound 1, the AHP's degree bounds); the index polynomials of ALL circuits are
+    then committed in one device pass (the reference commits circuit by circuit: the commitments are the same).  The commitments
+    are not blinded.  An SRS with fewer powers than a circuit's max_degree raises ValueError."""
+    srs_degree = pp_powers_of_beta_g.shape[0] - 1
+    keyed, bases, polys = [], [], []
+    for c in circuits:
+        info = c.info()
+        max_degree = info.max_degree(hiding)
+        if max_degree > srs_degree:
+            raise ValueError(f"the universal SRS supports degree {srs_degree}, the circuit needs {max_degree}")
+        ck = CommitterKey.trim(pp_powers_of_beta_g, pp_powers_of_beta_times_gamma_g, max_degree, (), 1, info.degree_bounds())
+        labeled = c.interpolate_matrix_evals()
+        keyed.append((c, info, ck, labeled))
+        bases += [ck.powers_of_beta_g] * len(labeled)
+        polys += [p.polynomial for p in labeled]
+    comms = device.sonic_commit_batch(bases, polys)
+    out = []
+    for i, (c, info, ck, labeled) in enumerate(keyed):
+        rows = comms[12 * i: 12 * i + 12]
+        order = sorted(range(12), key=lambda j: labeled[j].label)
+        vk = VerifyingKey(info, rows[order].copy(), c.id())
+        out.append((ProvingKey(vk, c, ck), vk))
+    return out
+
+
+def circuit_setup(pp_powers_of_beta_g: torch.Tensor, pp_powers_of_beta_times_gamma_g: torch.Tensor, circuit: Circuit, hiding: bool = False):
+    """Varuna::circuit_setup (varuna.rs:223-233) → (ProvingKey, VerifyingKey)"""
+    return batch_circuit_setup(pp_powers_of_beta_g, pp_powers_of_beta_times_gamma_g, [circuit], hiding)[0]
+
+
+def _certificate_challenges(challenges, count: int):
+    """the squeezed values of the certificate sponge: the last is the point, the combiners are 1 and the others (varuna.rs:245-251)"""
+    challenges = [int(x) % R_MOD for x in challenges]
+    if len(challenges) != count:
+        raise ValueError(f"{count} challenges expected, one per index commitment")
+    return challenges[-1], [1] + challenges[:-1]
+
+
+def prove_vk(pk: ProvingKey, vk: VerifyingKey, challenges, opening_challenges):
+    """Varuna::prove_vk (varuna.rs:236-276): opens Σ c_i·p_i over the sorted labels at the point (LC `circuit_check`) with
+    SonicKZG10.open_combinations.  `challenges`: the twelve squeezed values; `opening_challenges`: what open_combinations squeezes
+    (one combiner, then the discarded randomizer).  → the BatchLCProof's [(w, random_v)]."""
+    point, combiners = _certificate_challenges(challenges, len(vk.circuit_commitments))
+    labeled = pk.circuit.interpolate_matrix_evals()
+    lc = [("circuit_check", list(zip(combiners, sorted(p.label for p in labeled))))]
+    query_set = [("circuit_check", ("challenge", point))]
+    return SonicKZG10.open_combinations(pk.committer_key, lc, labeled, [Randomness() for _ in labeled], query_set, iter(opening_challenges))
+
+
+def evaluate_index_polynomials(circuit: Circuit, point: int, combiners):
+    """AHPForR1CS::evaluate_index_polynomials (ahp/indexer/indexer.rs:232-260): the twelve evaluations at `point` through the
+    Lagrange coefficients of each K_M, summed in one device pass without interpolating → (("circuit_check", [(combiner, label)]),
+    Σ combiner·evaluation) over the sorted labels."""
+    combiners = [int(x) % R_MOD for x in combiners]
+    if len(combiners) != 12:
+        raise ValueError("one combiner per index polynomial")
+    dev = circuit.a.vals.device
+    lagrange = [K.evaluate_all_lagrange_coefficients(point, dev) for K in circuit.non_zero_domains]
+    sums = device.index_arithmetize(circuit._csr(), [K.size for K in circuit.non_zero_domains], circuit.num_variables,
+                                    circuit.num_public, lagrange)
+    evals = dict(zip(index_polynomial_labels(circuit.id()), (_fr_mont_to_int(v) for v in sums.reshape(12, 4))))
+    terms, total = [], 0
+    for comb, label in zip(combiners, sorted(evals)):
+        terms.append((comb, label))
+        total += comb * evals[label]
+    return ("circuit_check", terms), total % R_MOD
+
+
+def verify_vk_evaluation(circuit: Circuit, vk: VerifyingKey, challenges):
+    """The half of Varuna::verify_vk (varuna.rs:280-311) that precedes check_combinations: the re-indexed circuit must have the key's
+    info and id (else ValueError, SNARKError::CircuitNotFound), then → (lc, point, evaluation)."""
+    if circuit.info() != vk.circuit_info or circuit.id() != vk.id:
+        raise ValueError("CircuitNotFound: the circuit does not match the verifying key")
+    point, combiners = _certificate_challenges(challenges, len(vk.circuit_commitments))
+    lc, evaluation = evaluate_index_polynomials(circuit, point, combiners)
+    return lc, point, evaluation
